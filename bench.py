@@ -4,6 +4,8 @@
 Contract (one JSON line on stdout from rank 0):
   python bench.py --gpus N --steps K --warmup W            (N>1 under torchrun)
   python bench.py --impl reference ...                     (CPU CG+AMG arm)
+  python bench.py ... --dump-outputs DIR                   (also write the last timed step's results
+                                                            as DIR/<name>.npy, see dump_outputs)
 
 Default workload = the configuration BASELINE.json's metric is quoted on, "10^7-node raster":
 3163 x 3163 synthetic resistance raster (R ~ U[1,10], seed 42; n = 10 004 569, nnz = 90 003 169),
@@ -73,8 +75,12 @@ def parse():
     ap.add_argument("--skip-direct", action="store_true")
     ap.add_argument("--cpu-sample", type=int, default=16, help="pairs per CPU step (one per core)")
     ap.add_argument("--ref-budget-s", type=float, default=330.0,
-                    help="--impl reference: wall budget of the timed steps")
+                    help="--impl reference: wall budget that bounds the warm-up steps after the first")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     c = CONFIGS[a.config]
     a.rows = a.rows or c["rows"]
     a.cols = a.cols or c["cols"]
@@ -88,6 +94,20 @@ def peaks():
     if os.path.isfile(p):
         return json.load(open(p))["hbm_gbs"], "measured (MEASURED_PEAKS.json)"
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_SAMPLE = 1 << 20        # entries kept of a longer output: a 10^7-node map becomes 8 MB in fp64
+
+
+def dump_outputs(path, arrays):
+    """Write each array as path/<name>.npy.  An array longer than DUMP_SAMPLE is cut to the same
+    seeded sample of its entries on every run, so runs with the same arguments compare entry for entry."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if a.size > DUMP_SAMPLE:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))]
+        np.save(os.path.join(path, f"{name}.npy"), a)
 
 
 def b_spmm(n, nnz, k, sv):
@@ -253,28 +273,29 @@ def run_reference(args):
     L, src, dst = workload(args, npairs)
     arm = CpuArm(L, src, dst, args.cpu_sample)
     t1, _, _ = arm.step()                                   # warm-up 1 (page-in, worker start)
-    # a 10^7-node solve takes ~10 s per core: keep the timed region inside the budget
-    steps = max(1, min(args.steps, int(args.ref_budget_s / max(t1, 1e-3))))
+    # a 10^7-node solve takes ~10 s per core: more warm-up only while the run stays inside the budget
     warm = 1
-    while warm < args.warmup and (args.warmup - warm + steps) * t1 < args.ref_budget_s:
+    while warm < args.warmup and (args.warmup - warm + args.steps) * t1 < args.ref_budget_s:
         arm.step(); warm += 1
     times, iters = [], None
-    for _ in range(steps):
-        t, _, iters = arm.step()
+    for _ in range(args.steps):
+        t, R, iters = arm.step()
         times.append(t)
     arm.close()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"resistances": R})
     wall = float(np.mean(times))
     value = arm.sample / wall
     line = {
         "impl": "reference", "metric": "pair_solves_per_sec", "value": value, "unit": "pair-solves/s",
-        "n_gpus": args.gpus, "steps": steps, "warmup": warm, "ms_per_step": wall * 1e3,
+        "n_gpus": args.gpus, "steps": args.steps, "warmup": warm, "ms_per_step": wall * 1e3,
         "higher_is_better": True, "scaling": args.scaling, "vs_baseline": None, "dtype": "f64", "data": "synthetic",
         "config": config_dict(args, L, npairs, max(world, args.gpus)),
         "cpu_baseline": {"value": value, "unit": "pair-solves/s", "cores": arm.sample, "kind": "port",
                          "sample": f"{arm.sample} of {len(src)} pairs per step, one pair per process on "
                                    f"{arm.host_cores} host cores (SA-AMG + symmetric-GS PCG rtol 1e-6, oracle/amg.py; "
                                    f"AMG setup {arm.setup_s:.1f}s excluded, levels {arm.levels}; iterations {iters}); "
-                                   f"steps/warm-up requested {args.steps}/{args.warmup}, bounded by --ref-budget-s"},
+                                   f"warm-up requested {args.warmup}, bounded by --ref-budget-s"},
         "setup": {"amg_setup_s": arm.setup_s,
                   "setup_inclusive_pair_solves_per_s": arm.sample / (arm.setup_s + wall)},
         "e2e": {"value": value, "unit": "pair-solves/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
@@ -429,6 +450,11 @@ def main():
     ms, wall, res = timed(step, args.steps)
     clocks = sampler.stop() if sampler else None
     R, out, st = res[-1]
+    if args.dump_outputs and rank == 0:
+        # what a caller of the step receives: every pair's resistance and the job's current maps
+        # (cumulative and max over pairs, summed / maxed over ranks); iterations and residuals are in the JSON line
+        cum, mx = factor.read_currents()
+        dump_outputs(args.dump_outputs, {"resistances": R, "cum_current": cum, "max_current": mx})
     launches = sum(r[2]["kernel_launches"] for r in res)
     iters = out["iters"]
     value = npairs * args.steps / (ms / 1e3)

@@ -29,21 +29,30 @@ _SO = os.path.join(_HERE, "_ref", "liboracle_amg.so")
 _lib = None
 
 
-def build(force=False):
-    """gcc -O3 the sequential kernels (called by __graft_entry__.build())."""
-    src = os.path.join(_HERE, "csrc", "amg_kernels.c")
-    os.makedirs(os.path.dirname(_SO), exist_ok=True)
-    if force or not os.path.isfile(_SO) or os.path.getmtime(_SO) < os.path.getmtime(src):
+_SRC = os.path.join(_HERE, "csrc", "amg_kernels.c")
+
+
+def _stale(so):
+    return not os.path.isfile(so) or os.path.getmtime(so) < os.path.getmtime(_SRC)
+
+
+def build(force=False, so=_SO):
+    """gcc -O3 the sequential kernels into `so` (called by __graft_entry__.build())."""
+    os.makedirs(os.path.dirname(so), exist_ok=True)
+    if force or _stale(so):
         import subprocess
-        subprocess.check_call(["gcc", "-O3", "-march=x86-64-v2", "-shared", "-fPIC", "-o", _SO, src])
-    return _SO
+        subprocess.check_call(["gcc", "-O3", "-march=x86-64-v2", "-shared", "-fPIC", "-o", so, _SRC])
+    return so
 
 
 def _load():
     global _lib
     if _lib is None:
-        build()
-        lib = C.CDLL(_SO)
+        so = _SO
+        if _stale(so):      # not built or out of date: compile a private copy, the source tree may be read-only
+            import tempfile
+            so = build(so=os.path.join(tempfile.mkdtemp(prefix="oracle_amg_"), "liboracle_amg.so"))
+        lib = C.CDLL(so)
         i32p, f64p = C.POINTER(C.c_int32), C.POINTER(C.c_double)
         lib.csr_matvec.argtypes = [C.c_int64, i32p, i32p, f64p, f64p, f64p]
         lib.gauss_seidel.argtypes = [C.c_int64, i32p, i32p, f64p, f64p, f64p, C.c_int]
