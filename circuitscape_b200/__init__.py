@@ -11,5 +11,5 @@ from .solver import (CUDAB200, CUDASolver, B200Factor, SolverResidualError,  # n
 from .core import (GraphProblem, AdvancedProblem, Flags, OutputFlags, get_solver,  # noqa: F401
                    single_ground_all_pairs, solve, advanced_kernel, multiple_solver, compute_3col,
                    RasterData, onetoall_kernel, resolve_conflicts, compute_omniscape_current,
-                   all_to_one_batched)
+                   all_to_one_batched, raster_pairwise)
 from ._lib import B200Unavailable, B200Error, LIB_PATH, EXPORTED_SYMBOLS  # noqa: F401

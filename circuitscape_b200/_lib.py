@@ -65,6 +65,7 @@ _PROTOS = {
     "cs_b200_create_from_raster_poly": (C.c_int, [C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                                   C.c_int, C.POINTER(Opts), C.POINTER(_H), C.POINTER(C.c_int64),
                                                   C.POINTER(C.c_int64), C.c_void_p]),
+    "cs_b200_components": (C.c_int, [_H, C.c_void_p, C.POINTER(C.c_int64)]),
     "cs_b200_get_dims": (C.c_int, [_H, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "cs_b200_destroy": (None, [_H]),
     "cs_b200_spmv": (C.c_int, [_H, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_double)]),

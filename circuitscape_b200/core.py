@@ -14,6 +14,7 @@ flags ask for) come back.
 """
 from __future__ import annotations
 
+import contextlib
 from dataclasses import dataclass, field
 
 import numpy as np
@@ -179,11 +180,34 @@ def single_ground_all_pairs(prob: GraphProblem, flags: Flags, cfg=None, log=True
     return solve(prob, prob.solver, flags, cfg, log, sink=sink)
 
 
-def solve(prob: GraphProblem, solver: S.CUDASolver, flags: Flags, cfg=None, log=True, sink=None) -> PairwiseOutput:
+def _component_rows(nodemap, comp, polymap, n):
+    """cell -> 1-based row of a whole-graph factor with n rows: the node whose value the component's
+    local node map puts in the cell (row l of the component's submatrix is node comp[l]; with polygons
+    the local numbering can differ from the submatrix's, and the maps follow the local numbering).
+    Without polygons that is the cell's own node wherever it lies in the component."""
+    if polymap is None or np.size(polymap) == 0:
+        member = np.zeros(n + 1, dtype=bool)
+        member[comp] = True
+        return np.where(member[nodemap], nodemap, 0)
+    lm = construct_local_node_map(nodemap, comp, polymap)
+    return np.where(lm != 0, comp[np.maximum(lm, 1) - 1], 0)
+
+
+def solve(prob: GraphProblem, solver: S.CUDASolver, flags: Flags, cfg=None, log=True, sink=None,
+          factor=None) -> PairwiseOutput:
     """`sink`: optional writer the per-pair results are handed to as each batch finishes -- the
     reference writes every map inside `postprocess` and drops it (src/core.jl:655-683); without a
     sink they are kept in the returned object (tests, small jobs).  A sink has the methods
-    `voltmap(key, grid)`, `curmap(key, grid)` (raster) and `network(key, comp, volt, cur, branch)`."""
+    `voltmap(key, grid)`, `curmap(key, grid)` (raster) and `network(key, comp, volt, cur, branch)`.
+
+    `factor`: one resident factor whose row r is node r + 1 of the whole graph, e.g. a whole-raster
+    handle (B200Factor.from_raster_polygons; block-diagonal over the components).  Every component's
+    pairs are solved on it instead of on a factor of the component's submatrix, and the cumulative /
+    max vectors are read back once for the job.  Raster mode only; `prob.G` is not used and
+    `prob.cc` only needs the components that hold a focal node.  The caller keeps ownership."""
+    shared = factor is not None
+    if shared and not flags.is_raster:
+        raise ValueError("solve(factor=...) serves raster problems only")
     o = flags.outputflags
     P = len(prob.points)
     R = -np.ones((P, P))
@@ -200,9 +224,15 @@ def solve(prob: GraphProblem, solver: S.CUDASolver, flags: Flags, cfg=None, log=
         out.cum_node = np.zeros(prob.G.shape[0])
         out.cum_branch = np.zeros(len(prob.coords[0]))
         branch_pos = _BranchIndex(prob.coords)
-    G = sp.csr_matrix(prob.G)
+    G = None if shared else sp.csr_matrix(prob.G)
     points = np.asarray(prob.points)
     ids = np.asarray(prob.user_points)
+    if shared:
+        factor.reset_currents()
+        local_of = np.arange(-1, factor.n, dtype=np.int64)      # node id -> row of the shared factor
+        rows_of_cells = np.asarray(prob.nodemap)                 # cell -> row + 1 read for the cumulative maps
+        has_polygons = prob.polymap is not None and np.size(prob.polymap) > 0
+        npost_total = 0.0
 
     for comp in prob.cc:
         comp = np.asarray(comp)
@@ -217,19 +247,25 @@ def solve(prob: GraphProblem, solver: S.CUDASolver, flags: Flags, cfg=None, log=
                 _update_shortcut_resistances(anchor, voltmatrix, shortcut_res, R, points, comp)
             continue
         rows = comp - 1
-        matrix = G[rows][:, rows].tocsr()
-        local_of = np.zeros(G.shape[0] + 1, dtype=np.int64)
-        local_of[comp] = np.arange(len(comp))
+        if not shared:
+            matrix = G[rows][:, rows].tocsr()
+            local_of = np.zeros(G.shape[0] + 1, dtype=np.int64)
+            local_of[comp] = np.arange(len(comp))
         src = np.array([local_of[s] for s, _, _ in solves])
         dst = np.array([local_of[d] for _, d, _ in solves])
         weight = np.array([len(f) for _, _, f in solves], dtype=np.float64)
         need_curr = not shortcut                       # postprocess always builds the current map
         per_pair_volt = o.write_volt_maps or (not raster and not shortcut)   # network branch currents need v
         per_pair_curr = need_curr and ((o.write_cur_maps and not o.write_cum_cur_map_only) or not raster)
-        local_nodemap = construct_local_node_map(prob.nodemap, comp, prob.polymap) if raster and not shortcut else None
+        local_nodemap = None
+        if raster and not shortcut and not shared:
+            local_nodemap = construct_local_node_map(prob.nodemap, comp, prob.polymap)
+        elif raster and not shortcut and (o.write_volt_maps or per_pair_curr or has_polygons):
+            local_nodemap = _component_rows(prob.nodemap, comp, prob.polymap, factor.n)
         # only raster maps are log-transformed (src/out.jl:96 process_grid!); the network branch of
         # write_cur_maps accumulates raw node currents (src/out.jl:48-88)
-        with S.construct_cholesky_factor(matrix, solver, log_transform=bool(o.log_transform_maps and raster)) as factor:
+        with (contextlib.nullcontext(factor) if shared else
+              S.construct_cholesky_factor(matrix, solver, log_transform=bool(o.log_transform_maps and raster))) as factor:
             bs = max(1, int(solver.bs))
             if shortcut:
                 inside = np.nonzero(np.isin(points, comp) & (points != 0))[0]
@@ -301,7 +337,11 @@ def solve(prob: GraphProblem, solver: S.CUDASolver, flags: Flags, cfg=None, log=
                                     out.voltmaps[key] = (comp, v)
                                 out.curmaps[key] = (comp, cur)
                                 out.branch[key] = br
-            if need_curr:
+            if need_curr and shared:
+                npost_total += float(weight.sum())
+                if has_polygons:
+                    rows_of_cells = np.where(local_nodemap != 0, local_nodemap, rows_of_cells)
+            elif need_curr:
                 cum, mx = factor.read_currents(want_max=True)
                 if raster:
                     npost = float(weight.sum())
@@ -324,6 +364,8 @@ def solve(prob: GraphProblem, solver: S.CUDASolver, flags: Flags, cfg=None, log=
         if shortcut:
             anchor = int(np.nonzero(points == csub[0])[0][0])
             _update_shortcut_resistances(anchor, voltmatrix, shortcut_res, R, points, comp)
+    if shared and npost_total > 0:
+        _add_whole_raster_currents(out, factor, rows_of_cells, npost_total, prob.cellmap, o)
     if shortcut:
         R = shortcut_res
     np.fill_diagonal(R, 0.0)
@@ -336,6 +378,105 @@ def solve(prob: GraphProblem, solver: S.CUDASolver, flags: Flags, cfg=None, log=
         out.cum_curmap = np.where(out.cum_curmap < NODATA, NODATA, out.cum_curmap)   # src/utils.jl:114-120
         if out.max_curmap is not None:
             out.max_curmap = np.where(out.max_curmap < NODATA, NODATA, out.max_curmap)
+    return out
+
+
+def _add_whole_raster_currents(out, factor, rows_of_cells, npost, cellmap, o):
+    """The cumulative / max maps of a job solved on one whole-raster factor, from ONE read of its
+    vectors.  Equal to the per-component sums of `solve` on per-component factors: a node outside a
+    pair's component carries zero current (the 1e-8 relative zeroing removes the coupling noise of
+    the coarse pseudo-inverse), which the log transform accumulates as NODATA once per post-processed
+    pair -- what the per-component path adds for cells outside each component; cells without a node
+    get NODATA times the job's count directly.  `rows_of_cells`: cell -> row + 1 (0 = no node)."""
+    cum, mx = factor.read_currents(want_max=True)
+    off = rows_of_cells == 0
+    cmap = _scatter(cum.astype(np.float64), rows_of_cells)
+    if o.log_transform_maps:
+        cmap = np.where(off, NODATA * npost, cmap)
+    if o.set_null_currents_to_nodata:
+        cmap = np.where(cellmap == 0, NODATA * npost, cmap)
+    out.cum_curmap += cmap
+    if out.max_curmap is not None:
+        mmap = np.where(off, NODATA if o.log_transform_maps else 0.0, _scatter(mx.astype(np.float64), rows_of_cells))
+        if o.set_null_currents_to_nodata:
+            mmap = np.where(cellmap == 0, NODATA, mmap)
+        out.max_curmap = np.maximum(out.max_curmap, mmap)
+
+
+def _focal_components(factor, points):
+    """Components (1-based node ids, ascending) of a whole-graph factor that hold a focal node, in order
+    of their smallest node, from the device labels (cs_b200_components)."""
+    labels, _ = factor.components()
+    pts = np.asarray(points, dtype=np.int64)
+    pts = pts[pts != 0]
+    return [np.flatnonzero(labels == c) + 1 for c in np.unique(labels[pts - 1])]
+
+
+def raster_pairwise(cellmap, points_rc, flags: Flags, polymap=None, exclude_pairs=frozenset(), solver=None,
+                    four_neighbors=False, avg_res=False, sink=None) -> PairwiseOutput:
+    """Raster pairwise job from the conductance raster (src/raster/pairwise.jl:14-135), assembled,
+    labelled and solved on the device.
+
+    cellmap: conductances after masking (cells <= 0 are not nodes); points_rc: (rows, cols, ids)
+    1-based, after include / exclude filtering; exclude_pairs: id pairs not to solve.  The output is
+    that of `single_ground_all_pairs` on the host-built problem (resistances with the id header,
+    per-pair maps or `sink`, cumulative / max maps, num_solves).
+
+    Unique focal ids: ONE whole-raster factor (node map, Laplacian and components built on the
+    device) serves every component's pairs.  Repeated ids (focal regions): one device assembly per
+    pair on that pair's polygon map, as the reference rebuilds its graph per pair."""
+    from . import graph
+    solver = solver if solver is not None else S.CUDASolver()
+    rr, cc_, ids = (np.asarray(a) for a in points_rc)
+    log_t = bool(flags.outputflags.log_transform_maps)
+
+    def run(poly, nodes, user_points, exclude):
+        f, nodemap = S.B200Factor.from_raster_polygons(cellmap, poly, solver, four_neighbors=four_neighbors,
+                                                       avg_res=avg_res, log_transform=log_t)
+        with f:
+            prob = GraphProblem(None, _focal_components(f, nodes(nodemap)), nodes(nodemap), user_points,
+                                set(exclude), nodemap, poly, cellmap, solver)
+            return solve(prob, solver, flags, sink=sink, factor=f)
+
+    if len(ids) == len(np.unique(ids)):
+        return run(polymap, lambda nm: nm[rr - 1, cc_ - 1], ids, exclude_pairs)
+
+    pts = list(dict.fromkeys(int(p) for p in ids))
+    first = {p: int(np.nonzero(ids == p)[0][0]) for p in pts}
+    n = len(pts)
+    R = -np.ones((n, n))
+    out = None
+    for i in range(n):
+        for j in range(i + 1, n):
+            p1, p2 = pts[i], pts[j]
+            if (p1, p2) in exclude_pairs or (p2, p1) in exclude_pairs:
+                continue
+            x, y = first[p1], first[p2]
+            r = run(graph.create_pair_polymap(cellmap, polymap, (rr, cc_, ids), p1, p2),
+                    lambda nm: np.array([nm[rr[x] - 1, cc_[x] - 1], nm[rr[y] - 1, cc_[y] - 1]]),
+                    np.array([p1, p2]), ())
+            R[i, j] = R[j, i] = r.resistances[1, 2]
+            if out is None:
+                out = r
+                continue
+            out.voltmaps.update(r.voltmaps)
+            out.curmaps.update(r.curmaps)
+            out.cum_curmap = out.cum_curmap + r.cum_curmap
+            if out.max_curmap is not None:
+                out.max_curmap = np.maximum(out.max_curmap, r.max_curmap)
+            out.num_solves += r.num_solves
+            out.iterations += r.iterations
+            out.stats += r.stats
+    if out is None:                                       # every pair excluded
+        out = PairwiseOutput(resistances=None, cum_curmap=np.zeros(np.shape(cellmap)),
+                             max_curmap=np.full(np.shape(cellmap), NODATA)
+                             if flags.outputflags.write_max_cur_maps else None)
+    np.fill_diagonal(R, 0.0)
+    full = np.zeros((n + 1, n + 1))
+    full[0, 1:] = pts
+    full[1:, 0] = pts
+    full[1:, 1:] = R
+    out.resistances = full
     return out
 
 

@@ -20,6 +20,7 @@
 #include "win_host.hpp"
 #include "kernels.cuh"
 #include "raster_assembly.cuh"
+#include "components.cuh"
 #include "setup_device.hpp"
 
 using namespace csb;
@@ -82,6 +83,7 @@ struct cs_b200_handle {
   void* d_vals = nullptr;
   bool owns_matrix = true;
   void* d_vals0 = nullptr;           // pristine values while grounds are applied (cs_b200_set_grounds)
+  bool grounds_applied = false;      // d_vals currently differ from the operator as created
   void* d_dinv = nullptr;
   int* d_bstart = nullptr;
   int nblocks = 0;
@@ -1866,7 +1868,7 @@ static void teardown_operators(cs_b200_handle* h) {
 
 extern "C" {
 
-int cs_b200_version(void) { return 1001; }
+int cs_b200_version(void) { return 1002; }
 
 const char* cs_b200_last_error(const cs_b200_handle* h) {
   return h ? h->err.c_str() : g_create_error.c_str();
@@ -2263,6 +2265,7 @@ int cs_b200_set_grounds(cs_b200_handle* h, const void* finite_g, const uint8_t* 
   if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
   cleanup();
   if (e != cudaSuccess) return set_err(h, CS_B200_ERR_CUDA, "CUDA error %s applying the grounds", cudaGetErrorString(e));
+  h->grounds_applied = finite_g || dirichlet;
   teardown_operators(h);
   const csb_dev::HostPattern none{};
   int rc = h->dtype == CS_B200_F64 ? build_operators<double>(h, none, nullptr, nullptr)
@@ -2273,6 +2276,52 @@ int cs_b200_set_grounds(cs_b200_handle* h, const void* finite_g, const uint8_t* 
   float ms = 0;
   cudaEventElapsedTime(&ms, h->ev0, h->ev1);
   h->stats.setup_ms = ms;
+  return CS_B200_OK;
+}
+
+int cs_b200_components(cs_b200_handle* h, int32_t* label, int64_t* ncomp) {
+  if (!h) return CS_B200_ERR_ARG;
+  if (!label) return set_err(h, CS_B200_ERR_ARG, "label is NULL");
+  if (h->grounds_applied)
+    return set_err(h, CS_B200_ERR_UNSUPPORTED, "cs_b200_components: grounds are applied (cs_b200_set_grounds)");
+  cudaSetDevice(h->device);
+  h->err.clear();
+  const int n = (int)h->n;
+  int *d_parent = nullptr, *d_flag = nullptr, *d_ord = nullptr;
+  auto cleanup = [&]() { cudaFree(d_parent); cudaFree(d_flag); cudaFree(d_ord); };
+#define CKC_(call)                                                                         \
+  do {                                                                                     \
+    cudaError_t _e = (call);                                                               \
+    if (_e != cudaSuccess) {                                                               \
+      cleanup();                                                                           \
+      return set_err(h, CS_B200_ERR_CUDA, "CUDA error %s at %s:%d (%s)",                   \
+                     cudaGetErrorString(_e), __FILE__, __LINE__, #call);                   \
+    }                                                                                      \
+  } while (0)
+  CKC_(cudaMalloc(&d_parent, (size_t)n * sizeof(int)));
+  CKC_(cudaMalloc(&d_flag, (size_t)(n + 1) * sizeof(int)));
+  CKC_(cudaMalloc(&d_ord, (size_t)(n + 1) * sizeof(int)));
+  CKC_(cudaMemsetAsync(d_flag + n, 0, sizeof(int), h->stream));   // ordinal[n] = number of components
+  const int grid = (int)std::min<int64_t>((h->n + 255) / 256, (int64_t)h->num_sms * 32);
+  if (h->dtype == CS_B200_F64) {
+    ccl::k_cc_init<double><<<grid, 256, 0, h->stream>>>(n, h->d_rowptr, h->d_colidx, (const double*)h->d_vals, d_parent);
+    ccl::k_cc_hook<double><<<grid, 256, 0, h->stream>>>(n, h->d_rowptr, h->d_colidx, (const double*)h->d_vals, d_parent);
+  } else {
+    ccl::k_cc_init<float><<<grid, 256, 0, h->stream>>>(n, h->d_rowptr, h->d_colidx, (const float*)h->d_vals, d_parent);
+    ccl::k_cc_hook<float><<<grid, 256, 0, h->stream>>>(n, h->d_rowptr, h->d_colidx, (const float*)h->d_vals, d_parent);
+  }
+  ccl::k_cc_flatten<<<grid, 256, 0, h->stream>>>(n, d_parent, d_flag);
+  CKC_(cudaGetLastError());
+  CKC_(ras::exclusive_scan(d_flag, d_ord, (int64_t)n + 1, h->stream));
+  ccl::k_cc_label<<<grid, 256, 0, h->stream>>>(n, d_parent, d_ord, d_flag);
+  CKC_(cudaGetLastError());
+  CKC_(cudaMemcpyAsync(label, d_flag, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  int total = 0;
+  CKC_(cudaMemcpyAsync(&total, d_ord + n, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  CKC_(cudaStreamSynchronize(h->stream));
+#undef CKC_
+  cleanup();
+  if (ncomp) *ncomp = total;
   return CS_B200_OK;
 }
 

@@ -64,6 +64,40 @@ def create_new_polymap(gmap, polymap, points_rc, point_map):
     return newpoly
 
 
+def create_pair_polymap(gmap, polymap, points_rc, pt1, pt2):
+    """Polygon map of one pair of focal REGIONS (pairwise with repeated focal ids,
+    src/raster/pairwise.jl:405-442): without a polygon map every cell of pt1 / pt2 becomes a polygon
+    named after its id; with one, a region of several cells that touches no polygon becomes a new
+    polygon, and one that touches polygons merges all of them into a new polygon."""
+    rr, cc, ids = (np.asarray(a) for a in points_rc)
+    if polymap is None or np.size(polymap) == 0:
+        newpoly = np.zeros(np.shape(gmap), dtype=np.int64)
+        for p in (pt1, pt2):
+            sel = ids == p
+            newpoly[rr[sel] - 1, cc[sel] - 1] = p
+        return newpoly
+    polymap = np.asarray(polymap, dtype=np.int64)
+    newpoly = polymap.copy()
+    k = int(polymap.max())
+    for p in (pt1, pt2):
+        idx = np.nonzero(ids == p)[0]
+        if len(idx) == 1:
+            continue
+        under = polymap[rr[idx] - 1, cc[idx] - 1]
+        if np.all(under == 0):
+            newpoly[rr[idx] - 1, cc[idx] - 1] = k + 1
+            k += 1
+            continue
+        touched = under[under != 0]
+        if len(touched) == 1:
+            # the reference reads an undefined variable (`overlap`) on this branch and stops there
+            raise ValueError(f"focal region {p} overlaps a short-circuit polygon in exactly one cell: "
+                             "the reference cannot build its polygon map (UndefVarError)")
+        newpoly[np.isin(polymap, touched)] = k + 1
+        k += 1
+    return newpoly
+
+
 def construct_graph(gmap, nodemap, avg_res, four_neighbors):
     """Symmetric adjacency of conductances: E, S, SE, NE neighbours, duplicates
     (parallel cell adjacencies of merged nodes) summed."""

@@ -174,6 +174,15 @@ class B200Factor:
         _lib.check(self._lib, self._h, self._lib.cs_b200_get_csr(self._h, _lib._ptr(rp), _lib._ptr(ci), _lib._ptr(va)))
         return sp.csr_matrix((va, ci, rp), shape=(n.value, n.value))
 
+    def components(self):
+        """cs_b200_components: (labels int32[n], ncomp) -- the 0-based component of every row of the
+        operator as created, components numbered in order of their smallest node (the order of
+        graph.connected_components)."""
+        lab = np.empty(self.n, dtype=np.int32)
+        ncomp = C.c_int64()
+        _lib.check(self._lib, self._h, self._lib.cs_b200_components(self._h, _lib._ptr(lab), C.byref(ncomp)))
+        return lab, ncomp.value
+
     def levels(self):
         """The multigrid hierarchy as SciPy matrices (downloaded; parity / debugging hook):
         list of dicts with A, P, R (None on the coarsest level), omega, windowed flags."""

@@ -166,6 +166,16 @@ int cs_b200_level_info(cs_b200_handle* h, int level, int which, int64_t* nrows, 
 int cs_b200_level_csr(cs_b200_handle* h, int level, int which, int32_t* rowptr, int32_t* colidx,
                       double* vals);
 
+/* Connected components of the handle's operator as created: an edge is a stored off-diagonal entry with
+ * a non-zero value. label: host, n int32, the 0-based ordinal of each node's component. Components are
+ * numbered in order of their smallest node: the order of graph.connected_components and of
+ * Graphs.connected_components. Isolated nodes are components of their own. *ncomp may be NULL.
+ * Returns CS_B200_ERR_UNSUPPORTED on a handle with grounds applied (cs_b200_set_grounds).
+ * Union-find on the device (hooking with path halving, then one prefix sum over the root flags); with
+ * the whole-raster handles of cs_b200_create_from_raster[_poly] this says which pairs a solve may
+ * take (both nodes in one component) without building the graph on the host.                       */
+int cs_b200_components(cs_b200_handle* h, int32_t* label, int64_t* ncomp);
+
 /* n and nnz of the handle's operator. */
 int cs_b200_get_dims(const cs_b200_handle* h, int64_t* n, int64_t* nnz);
 
